@@ -169,6 +169,24 @@ def cpu_oracle(max_frames, budget_s):
     return fps, len(frames), threads or 0, note
 
 
+DUMP_BUDGET_BYTES = 64 << 20
+
+
+def dump_outputs(arrays, out_dir, budget=DUMP_BUDGET_BYTES):
+    """write {name: tensor} as out_dir/<name>.npy in float32 (float64 stays float64).  When the whole set exceeds `budget`
+    bytes, every array larger than its even share is replaced by a fixed sample: the flat elements at indices drawn without
+    replacement from a generator seeded by the array's size, in ascending order, so two runs sample the same elements."""
+    import numpy as np
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items()}
+    arrays = {k: v if v.dtype == np.float64 else v.astype(np.float32) for k, v in arrays.items()}
+    total, share = sum(v.nbytes for v in arrays.values()), budget // max(1, len(arrays))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in sorted(arrays.items()):
+        if total > budget and v.nbytes > share:
+            v = v.reshape(-1)[np.sort(np.random.default_rng(v.size).choice(v.size, size=share // v.itemsize, replace=False))]
+        np.save(os.path.join(out_dir, k + '.npy'), v)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -185,7 +203,12 @@ def main():
                     help='dense-conv engine: tcgen05 scaled-split fp16 (fp32-class, default), tcgen05 3xTF32, single-pass TF32, or SIMT fp32')
     ap.add_argument('--dbg', type=int, default=0, help='experiment: tt_debug_set knob bits (see csrc/gemm_conv_tc.cu)')
     ap.add_argument('--tc-reserve', type=int, default=0, help='experiment: SMs the persistent tcgen05 kernels leave free for the side branch')
+    ap.add_argument('--dump-outputs', default=None, metavar='DIR',
+                    help='write the prediction dict of the last timed step (inputs resident) as DIR/<name>.npy (rank 0; <= 64 MB in '
+                         'all, larger arrays replaced by a fixed seeded sample, see dump_outputs)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     rank, world = int(os.environ.get('RANK', 0)), int(os.environ.get('WORLD_SIZE', 1))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))
 
@@ -238,9 +261,11 @@ def main():
     resident = {k: (v.to(dev) if torch.is_tensor(v) else v) for k, v in host.items()}
     from thinktwice_b200.parallel import gather_waypoints
     gathered = torch.empty(world * B, 6, 4, 2, device=dev) if world > 1 else None
+    last = {}
 
     def step(batch):
         pred = model.forward_inference(batch)
+        last['pred'] = pred
         wp = pred['pred_wp']
         if world > 1:                                            # the path's single collective: gather of the waypoints
             return gather_waypoints(wp, world, out=gathered)
@@ -279,6 +304,9 @@ def main():
     th = threading.Thread(target=clocks_sampler, args=(stop, samples, local_rank), daemon=True)
     th.start()
     ms = timed(resident, args.steps, read_back=False)
+    if args.dump_outputs and rank == 0:                          # before the next forward: the bulky outputs are views of the arena
+        pred = last['pred']
+        dump_outputs({k: pred[k] for k in pred.keys()}, args.dump_outputs)
     launches = launches_per_step * args.steps                    # graph replays execute the same kernel nodes every step
     for _ in range(max(args.warmup, 3)):                         # the host-input path has its own graphs / buffers: warm them outside the timed region
         step(host).cpu()

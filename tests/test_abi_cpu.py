@@ -58,20 +58,17 @@ def test_product_fails_loudly_without_cuda():
 
 
 def test_config_model_section_equals_reference_when_present():
+    """the model section of configs/thinktwice.py carries the reference's values: compared with the reference's own model
+    section, stored as tests/golden/ref_config_model.json (make_reference_checks_golden.py)."""
+    import json
+    import sys
     from thinktwice_b200.config import Config, DEFAULT_CONFIG
-    ref_path = '/root/reference/open_loop_training/configs/thinktwice.py'
+    sys.path.insert(0, os.path.join(ROOT, 'tests', 'golden'))
+    from make_reference_checks_golden import norm_config as norm
     ours = Config.fromfile(DEFAULT_CONFIG)
     assert ours.model.decoder.config.pred_len == 4 and ours.model.img_encoder.final_dim == (448, 896)
-    if not os.path.exists(ref_path):
-        return
-    ref = Config.fromfile(ref_path)
-
-    def norm(x):
-        if isinstance(x, dict):
-            return {k: norm(v) for k, v in x.items()}
-        if isinstance(x, (list, tuple)):
-            return [norm(v) for v in x]
-        return x
+    with open(os.path.join(ROOT, 'tests', 'golden', 'ref_config_model.json')) as f:
+        ref = json.load(f)
 
     def diff(a, b, path=''):
         out = []
@@ -81,7 +78,7 @@ def test_config_model_section_equals_reference_when_present():
         elif a != b:
             out.append((path, a, b))
         return out
-    assert not diff(norm(ours.model), norm(ref.model))
+    assert not diff(norm(ours.model), ref)
 
 
 def test_ctypes_structs_match_the_c_header(tmp_path):

@@ -125,106 +125,74 @@ def test_oracle_forward_inference_equals_the_reference_end_to_end(seed):
         assert rel(pred[k].numpy(), f[k]) < 1e-5, k
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/open_loop_training/code'), reason='needs the mounted reference tree')
 @pytest.mark.parametrize('seed', [0, 1, 2])
 def test_committed_plumbing_golden_is_reproduced_by_the_reference_code(seed):
-    """tests/golden/plumbing_seed*.npz (what the GPU suite holds the product to) were generated by the oracle; here the SAME
-    calibrated weights are loaded into the reference's own EncoderDecoder (reference framework + LSS + decoder behind import
-    stubs, state_dict names identical) and its forward_inference must give the stored vectors — so the GPU golden test is,
-    transitively, a test against the reference's code.  Runs only where /root/reference is mounted (the build container)."""
-    import make_reference_golden as mg
-    from oracle.lidar import LidarNet
+    """tests/golden/plumbing_seed*.npz (what the GPU suite holds the product to) were generated by the oracle; the reference's own
+    EncoderDecoder.forward_inference (reference framework + LSS + decoder behind import stubs, state_dict names identical) with the
+    SAME calibrated weights gave tests/golden/ref_calibrated_plumbing_seed*.npz (make_reference_checks_golden.py).  The committed
+    golden and the oracle run now must both equal it — so the GPU golden test is, transitively, a test against the reference's code."""
+    from make_reference_checks_golden import CALIBRATED_KEYS
     from oracle.model import EncoderDecoder as Oracle, calibrate_bn, init_oracle_weights
     from thinktwice_b200.config import Config, PLUMBING_CONFIG
     from thinktwice_b200.synthetic import make_batch
     cfg = Config.fromfile(PLUMBING_CONFIG)
-    mc = cfg.model
-    if 'olt_code.encoder_decoder_framework' in sys.modules:
-        fw, regs = sys.modules['olt_code.encoder_decoder_framework'], mg._REGS
-    else:
-        fw, regs = mg.load_reference()
-        mg.load_reference_lss(regs)
-        mg._REGS = regs
-    lss = sys.modules['olt_code.model_code.backbones.lss']
-    regs['BACKBONES'].classes['LSS'], regs['BACKBONES'].classes['LidarNet'] = lss.LSS, LidarNet
-    o = Oracle(**{k: v for k, v in mc.items() if k != 'type'})
+    o = Oracle(**{k: v for k, v in cfg.model.items() if k != 'type'})
     init_oracle_weights(o, seed)
     batch = make_batch(cfg, 1, seed=seed, num_points=2000)
     calibrate_bn(o, batch)
-    ref = fw.EncoderDecoder(img_encoder=dict(mc['img_encoder']), decoder=dict(mc['decoder']), lidar_encoder=dict(mc['lidar_encoder']),
-                            train_cfg=mc['train_cfg'], test_cfg=mc.get('test_cfg')).eval()
-    ref.load_state_dict(o.state_dict())                                # strict: identical names and shapes
-    batch['target_command_raw'] = batch['target_command'].argmax(-1)
     with torch.no_grad():
-        pred = ref.forward_inference(batch)
+        pred = o.eval().forward_inference(batch)
+    ref = np.load(os.path.join(G, f'ref_calibrated_plumbing_seed{seed}.npz'))
     g = np.load(os.path.join(G, f'plumbing_seed{seed}.npz'))
-    for k in ('pred_wp', 'mu_branches', 'sigma_branches', 'future_mu', 'future_sigma', 'pred_speed', 'pred_value_traj',
-              'refine_flattned_BEV_feature'):
-        assert rel(pred[k].numpy(), g[k]) < 1e-5, k
+    for k in CALIBRATED_KEYS:
+        assert rel(g[k], ref[k]) < 1e-5, k
+        assert rel(pred[k].numpy(), ref[k]) < 1e-5, k
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/open_loop_training/code'), reason='needs the mounted reference tree')
 def test_full_thinktwice_config_oracle_equals_the_reference_code():
     """the bench workload itself (thinktwice.py: 4 cams x 2 sweeps 448x896, 40k LiDAR points, K = 5, B = 1): the reference's
-    EncoderDecoder.forward_inference (its framework, LSS and decoder code; LiDAR encoder = oracle stand-in) against the oracle with
-    the same calibrated weights.  ~70 s of CPU."""
-    import make_reference_golden as mg
-    from oracle.lidar import LidarNet
+    EncoderDecoder.forward_inference (its framework, LSS and decoder code; LiDAR encoder = oracle stand-in) with the same calibrated
+    weights, as stored in tests/golden/ref_full_thinktwice.npz, against the oracle.  ~70 s of CPU."""
+    from make_reference_checks_golden import FULL_SHAPE_THREADS, fixed_threads, pred_digest
     from oracle.model import EncoderDecoder as Oracle, calibrate_bn, init_oracle_weights
     from thinktwice_b200.config import Config, DEFAULT_CONFIG
     from thinktwice_b200.synthetic import make_batch
     cfg = Config.fromfile(DEFAULT_CONFIG)
-    mc = cfg.model
-    if 'olt_code.encoder_decoder_framework' in sys.modules:
-        fw, regs = sys.modules['olt_code.encoder_decoder_framework'], mg._REGS
-    else:
-        fw, regs = mg.load_reference()
-        mg.load_reference_lss(regs)
-        mg._REGS = regs
-    lss = sys.modules['olt_code.model_code.backbones.lss']
-    regs['BACKBONES'].classes['LSS'], regs['BACKBONES'].classes['LidarNet'] = lss.LSS, LidarNet
-    o = Oracle(**{k: v for k, v in mc.items() if k != 'type'})
+    o = Oracle(**{k: v for k, v in cfg.model.items() if k != 'type'})
     init_oracle_weights(o, 0)
     batch = make_batch(cfg, 1, seed=0, num_points=40000)
-    calibrate_bn(o, batch)
-    ref = fw.EncoderDecoder(img_encoder=dict(mc['img_encoder']), decoder=dict(mc['decoder']), lidar_encoder=dict(mc['lidar_encoder']),
-                            train_cfg=mc['train_cfg'], test_cfg=mc.get('test_cfg')).eval()
-    ref.load_state_dict(o.state_dict())
-    batch['target_command_raw'] = batch['target_command'].argmax(-1)
-    with torch.no_grad():
-        pr, po = ref.forward_inference(batch), o.forward_inference(batch)
-    for k in mg.PRED_KEYS:
-        assert rel(po[k].numpy(), pr[k].numpy()) < 1e-6, k
+    with fixed_threads(FULL_SHAPE_THREADS):
+        calibrate_bn(o, batch)
+        with torch.no_grad():
+            po = pred_digest(o.eval().forward_inference(batch))
+    ref = np.load(os.path.join(G, 'ref_full_thinktwice.npz'))
+    assert sorted(po) == sorted(ref.files)
+    for k, v in po.items():
+        assert rel(v.numpy(), ref[k]) < 1e-6, k
 
 
-@pytest.mark.skipif(not os.path.isdir('/root/reference/open_loop_training/code'), reason='needs the mounted reference tree')
 @pytest.mark.parametrize('which', ['plumbing', 'full'])
 def test_product_host_camera_geometry_equals_the_reference_lss(which):
     """what the PRODUCT computes on the host for the camera branch (thinktwice_b200/lss.py: frustum axes, build_mats, the
     [ida^-1 | sensor2ego . intrin^-1] pair the lift kernel consumes, DepthNet's 22 camera scalars, the voxel-grid lower bound)
-    against the reference LSS: create_frustum, get_geometry (incl. transpose-not-inverse and key-frame mats for the history
-    sweep) and the tensor DepthNet feeds its BatchNorm1d(22)."""
-    import make_reference_golden as mg
+    against the reference LSS, as stored in tests/golden/ref_camera_geometry_*.npz: create_frustum, get_geometry (incl.
+    transpose-not-inverse and key-frame mats for the history sweep, at a seeded sample of frustum positions) and the tensor
+    DepthNet feeds its BatchNorm1d(22)."""
+    from make_reference_checks_golden import frustum_from_axes
     from thinktwice_b200.config import Config, DEFAULT_CONFIG, PLUMBING_CONFIG
     from thinktwice_b200.registry import BACKBONES
     from thinktwice_b200.synthetic import make_batch
     cfg = Config.fromfile(PLUMBING_CONFIG if which == 'plumbing' else DEFAULT_CONFIG)
-    if 'olt_code.encoder_decoder_framework' not in sys.modules:
-        _, regs = mg.load_reference()
-        mg.load_reference_lss(regs)
-        mg._REGS = regs
-    lss = sys.modules['olt_code.model_code.backbones.lss']
-    kw = {k: v for k, v in dict(cfg.model['img_encoder']).items() if k != 'type'}
-    ref = lss.LSS(**kw).eval()
+    ref = {k: torch.from_numpy(v) for k, v in np.load(os.path.join(G, f'ref_camera_geometry_{which}.npz')).items()}
     prod = BACKBONES.build(dict(cfg.model['img_encoder']))
     B = 2
     batch = make_batch(cfg, B, seed=3, num_points=10)
     metas = batch['img_metas']
     N = batch['img'].shape[2]
     # frustum and grid constants
-    assert torch.equal(prod.frustum, ref.frustum)
-    assert torch.equal(prod.voxel_coord - prod.voxel_size / 2.0, ref.voxel_coord - ref.voxel_size / 2.0)
-    assert [int(v) for v in prod.voxel_num] == [int(v) for v in ref.voxel_num]
+    assert torch.equal(prod.frustum, frustum_from_axes(ref['frustum.u'], ref['frustum.v'], ref['frustum.d']))
+    assert torch.equal(prod.voxel_coord - prod.voxel_size / 2.0, ref['lower'])
+    assert [int(v) for v in prod.voxel_num] == [int(v) for v in ref['voxel_num']]
     # matrices as LSS.forward assembles them (lss.py:667-687)
     mats = prod.build_mats(metas, N)
     intr = torch.stack([torch.stack([torch.cat([torch.cat([m['cam_intrinsic'], torch.zeros(N, 3, 1)], 2),
@@ -232,24 +200,18 @@ def test_product_host_camera_geometry_equals_the_reference_lss(which):
     assert torch.equal(mats['intrin_mats'], intr.float())
     # geometry: reference get_geometry vs the product's two matrices applied the way the lift kernel does
     T = len(metas[0])
-    fr = prod.frustum                                                  # (D, fH, fW, 4) = (u, v, d, 1)
+    fr = prod.frustum.reshape(-1, 4)[ref['sample_index']]             # (S, 4) = (u, v, d, 1) at the stored positions
     for s in range(T):
         idx = -1 if s == 0 else -s                                     # the sweep index LSS.forward passes (lss.py:689, 712)
-        geom_ref = ref.get_geometry(mats['sensor2ego_mats'][:, idx], mats['intrin_mats'][:, idx], mats['ida_mats'][:, idx], None)
+        geom_ref = ref[f'geom_mats{idx}']
         ida_inv = torch.inverse(mats['ida_mats'][:, idx])
         comb = mats['sensor2ego_mats'][:, idx].matmul(torch.inverse(mats['intrin_mats'][:, idx]))
-        p = torch.einsum('bnij,dhwj->bndhwi', ida_inv, fr)
+        p = torch.einsum('bnij,sj->bnsi', ida_inv, fr)
         p = torch.cat([p[..., :2] * p[..., 2:3], p[..., 2:]], -1)
-        geom = torch.einsum('bnij,bndhwj->bndhwi', comb, p)[..., :3]
+        geom = torch.einsum('bnij,bnsj->bnsi', comb, p)[..., :3]
         assert rel(geom.numpy(), geom_ref.numpy()) < 1e-6
         # and the integer voxel index, truncation toward zero (lss.py:630-631)
-        lower = ref.voxel_coord - ref.voxel_size / 2.0
-        assert torch.equal(((geom - lower) / ref.voxel_size).int(), ((geom_ref - lower) / ref.voxel_size).int())
-    # DepthNet's camera-awareness vector (lss.py:206-231): capture what reaches BatchNorm1d(22)
-    seen = {}
-    h = ref.depth_net.bn.register_forward_pre_hook(lambda m, inp: seen.setdefault('x', inp[0].detach().clone()))
-    with torch.no_grad():
-        x = torch.zeros(B * N, kw['depth_net_conf']['in_channels'], 2, 2)
-        ref.depth_net(x, {k: v for k, v in mats.items()})
-    h.remove()
-    assert torch.equal(prod.depthnet_mlp_input(mats)[:, :22], seen['x'].reshape(B * N, 22))
+        lower = ref['lower']
+        assert torch.equal(((geom - lower) / ref['voxel_size']).int(), ((geom_ref - lower) / ref['voxel_size']).int())
+    # DepthNet's camera-awareness vector (lss.py:206-231): what reaches BatchNorm1d(22)
+    assert torch.equal(prod.depthnet_mlp_input(mats)[:, :22], ref['depthnet_bn_input'])
